@@ -15,6 +15,8 @@ configs[2]).  The JSON line carries
 `--impl reference` times the CPU arm alone (oracle/_ref = the reference's own sources when they
 compiled here, else the oracle port).  Under torchrun (N > 1) the volume is sharded by coarse
 cell across ranks (strong scaling: every rank sees every frame and fuses its own cells).
+`--dump-outputs DIR` writes the volume the timed steps left behind (see dump_outputs) so that two
+builds can be compared output for output: the inputs are seeded, identical from run to run.
 """
 from __future__ import annotations
 
@@ -141,6 +143,22 @@ def bind_to_gpu_numa(gpu):
     return "default"
 
 
+DUMP_NODES = 1 << 20       # sampled nodes: 12 float32 values each = 48 MiB of .npy files
+
+
+def dump_outputs(out_dir, nodes, n_updates):
+    """What a caller of the timed path reads back after its last step, as float32 .npy files: every node array of the
+    volume's node dump (keys = level, x, y, z; {sdf, weight}; split flag; rgb; variance state) at a fixed, seeded sample of
+    DUMP_NODES node indices (every node when there are fewer; the dump is in octree order), and summary.npy = [number of
+    nodes, voxel updates of the last frame].  Every integer written is below 2^24, so float32 holds it exactly."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(nodes["keys"])
+    idx = np.arange(n) if n <= DUMP_NODES else np.sort(np.random.default_rng(0).choice(n, DUMP_NODES, replace=False))
+    for name in ("keys", "dw", "split", "rgb", "M", "ns"):
+        np.save(os.path.join(out_dir, name + ".npy"), nodes[name][idx].astype(np.float32))
+    np.save(os.path.join(out_dir, "summary.npy"), np.array([n, n_updates], np.float64))
+
+
 def oracle_volume(kind):
     from oracle.oracle_py import OracleVolume
     return OracleVolume(kind=kind, xres=RES, yres=RES, zres=RES, xsize=SIZE, ysize=SIZE, zsize=SIZE,
@@ -224,6 +242,8 @@ def run_reference(args, rank, world):
             v.integrate(clouds[k % ND], poses[k % ND]); k += 1
     dt = time.perf_counter() - t0
     fps = args.steps * frames_per_step / dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, v.dump_nodes(), v.stats().n_add_observation)
     line = {
         "impl": "reference", "metric": "integrateCloud frames/s @ 640x480 into 2048^3", "value": fps, "unit": "frames/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * dt / args.steps,
@@ -255,10 +275,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-host-load", action="store_true", help="skip the leg that repeats the device-resident measurement with all host cores busy")
     ap.add_argument("--pool-log2", type=int, default=18, help="brick pool capacity = 2^N slots (the bench scene allocates ~37k bricks)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the volume they left as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs needs a single rank: each rank of a sharded run holds only its own cells")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return
@@ -346,6 +369,8 @@ def main():
     prof, ms_total = timed(step_device, args.steps)
     nframes = args.steps * FRAMES_PER_STEP
     value = nframes / (ms_total / 1e3)
+    if args.dump_outputs:                                      # before the legs below integrate more frames into the volume
+        dump_outputs(args.dump_outputs, vol.download_nodes(), vol.stats().n_updates)
 
     # ---- the same work one frame per call, the dominant kernel bracketed by CUDA events (roofline leg) ----
     for _ in range(2):
@@ -379,7 +404,7 @@ def main():
         with (HostLoad(os.cpu_count() or 1) if rank == 0 else contextlib.nullcontext()):
             step_device(k); k += FRAMES_PER_STEP
             vol.sync()
-            n_loaded = max(16, args.steps)
+            n_loaded = args.steps
             loaded = []
             for _ in range(3):                                 # three repeats: a descheduled submitting thread shows as an outlier, not as the figure
                 _, ms_loaded = timed(step_device, n_loaded)

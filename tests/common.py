@@ -1,6 +1,8 @@
 """Shared helpers for the parity tests."""
 from __future__ import annotations
 
+import hashlib
+
 import numpy as np
 
 from cpu_tsdf_b200 import synth
@@ -30,6 +32,21 @@ def assert_same_nodes(a, b, *, rgb=False, var=False):
         assert np.array_equal(a["rgb"], b["rgb"]), "per-node rgb differs"
     if var:
         assert np.array_equal(a["M"].view(np.uint32), b["M"].view(np.uint32)) and np.array_equal(a["ns"], b["ns"])
+
+
+def sha(*arrays):
+    """SHA-256 of the arrays' bytes: equal digests = bit-identical arrays."""
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def sha_values(a):
+    """Digest under np.array_equal(..., equal_nan=True): every NaN is the same value, and -0.0 equals 0.0."""
+    a = np.asarray(a)
+    nan = np.isnan(a)
+    return sha(nan, np.where(nan, 0, a) + 0)
 
 
 def canon_soup(verts, cols=None):

@@ -1,15 +1,16 @@
 """Pins oracle/prog_oracle.cpp (the restatement of the reference's program-side functions) to the reference's OWN text of
-src/prog/integrate.cpp, compiled from the source where it lies (oracle/Makefile `refprog`: meshToFaceCloud, flattenVertices,
-cleanupMesh, reprojectPoint, lines 63-222; the per-cloud preparation + z-buffer re-organisation of main(), lines 559-635).
-Needs oracle/_ref/libcpu_tsdf_refprog.so, which only a container with /root/reference can build; the built file travels."""
-import os
+src/prog/integrate.cpp (meshToFaceCloud, flattenVertices, cleanupMesh, reprojectPoint, lines 63-222; the per-cloud preparation
++ z-buffer re-organisation of main(), lines 559-635).
 
+Each test compares what the restatement computes with what the same inputs gave through that text, compiled from the source
+where it lies (oracle/Makefile `refprog`).  Those results (SHA-256 digests of every compared array, and the counts) are stored in
+tests/golden/ref_pins.json; tools/make_ref_pins.py regenerates them where the reference sources are available."""
 import numpy as np
 import pytest
 
 from oracle import oracle_py
-
-pytestmark = pytest.mark.skipif(not os.path.exists(oracle_py.REFPROG_LIB), reason="oracle/_ref/libcpu_tsdf_refprog.so not built (needs /root/reference)")
+from tests.common import sha
+from tests.test_ref_pin import golden
 
 
 def _cloud(rng, n, spread=1.0):
@@ -22,8 +23,10 @@ def _cloud(rng, n, spread=1.0):
     return pts
 
 
-@pytest.mark.parametrize("seed,units,zero_nans,world", [(1, 1.0, False, False), (2, 0.001, True, False), (3, 1.0, True, True), (4, 2.5, False, True)])
-def test_organise_block_matches_the_reference_text(seed, units, zero_nans, world):
+ORGANISE_CASES = [(1, 1.0, False, False), (2, 0.001, True, False), (3, 1.0, True, True), (4, 2.5, False, True)]
+
+
+def observe_organise(kind, seed, units, zero_nans, world):
     rng = np.random.default_rng(seed)
     W, H = 160, 120
     intr = (131.25, 131.25, 79.5, 59.5)
@@ -38,12 +41,15 @@ def test_organise_block_matches_the_reference_text(seed, units, zero_nans, world
     if world:
         a = 0.3 * seed
         tf = np.array([[np.cos(a), 0, np.sin(a), 0.1], [0, 1, 0, -0.05], [-np.sin(a), 0, np.cos(a), 0.2], [0, 0, 0, 1]], np.float64)
-    kw = dict(rgba_off=16, cloud_units=units, zero_nans=zero_nans, world_to_camera=tf)
-    a, na = oracle_py.organize(pts, intr, W, H, kind="reference", **kw)
-    b, nb = oracle_py.organize(pts, intr, W, H, kind="port", **kw)
-    assert na == nb > 500
+    out, filled = oracle_py.organize(pts, intr, W, H, rgba_off=16, cloud_units=units, zero_nans=zero_nans, world_to_camera=tf, kind=kind)
+    assert filled > 500
     # x, y, z and the colour word; the padding float and the bytes after the colour are whatever the default point holds
-    assert np.array_equal(a.view(np.uint32)[..., :3], b.view(np.uint32)[..., :3]) and np.array_equal(a.view(np.uint32)[..., 4], b.view(np.uint32)[..., 4])
+    return {"filled": filled, "xyz": sha(out.view(np.uint32)[..., :3]), "rgba": sha(out.view(np.uint32)[..., 4])}
+
+
+@pytest.mark.parametrize("seed,units,zero_nans,world", ORGANISE_CASES)
+def test_organise_block_matches_the_reference_text(seed, units, zero_nans, world):
+    assert observe_organise("port", seed, units, zero_nans, world) == golden(f"organise[{seed}]")
 
 
 def _mc_like_mesh(rng, n_quads, jitter):
@@ -66,22 +72,50 @@ def _mc_like_mesh(rng, n_quads, jitter):
     return soup, np.arange(len(soup), dtype=np.int32).reshape(-1, 3)
 
 
-@pytest.mark.parametrize("seed,jitter,min_dist", [(1, 0.0, 1e-4), (2, 3e-5, 1e-4), (3, 2e-4, 2e-3), (4, 0.0, 0.0)])
-def test_flatten_vertices_matches_the_reference_text(seed, jitter, min_dist):
+def mesh_digests(v, t):
+    return {"n_verts": len(v), "n_tris": len(t), "verts": sha(v.view(np.uint32)), "tris": sha(t)}
+
+
+FLATTEN_CASES = [(1, 0.0, 1e-4), (2, 3e-5, 1e-4), (3, 2e-4, 2e-3), (4, 0.0, 0.0)]
+
+
+def observe_flatten(kind, seed, jitter, min_dist):
     rng = np.random.default_rng(seed)
     v, t = _mc_like_mesh(rng, 900, jitter)
-    va, ta = oracle_py.flatten_vertices(v, t, min_dist, kind="reference")
-    vb, tb = oracle_py.flatten_vertices(v, t, min_dist, kind="port")
-    assert len(va) == len(vb) and len(ta) == len(tb) and (min_dist == 0.0 or len(va) < len(v))
-    assert np.array_equal(va.view(np.uint32), vb.view(np.uint32)) and np.array_equal(ta, tb)
+    fv, ft = oracle_py.flatten_vertices(v, t, min_dist, kind=kind)
+    assert min_dist == 0.0 or len(fv) < len(v)
+    return mesh_digests(fv, ft)
 
 
-@pytest.mark.parametrize("seed,face_dist,min_neighbors", [(1, 0.02, 5), (2, 0.008, 3), (3, 0.05, 40)])
-def test_cleanup_mesh_matches_the_reference_text(seed, face_dist, min_neighbors):
+@pytest.mark.parametrize("seed,jitter,min_dist", FLATTEN_CASES)
+def test_flatten_vertices_matches_the_reference_text(seed, jitter, min_dist):
+    assert observe_flatten("port", seed, jitter, min_dist) == golden(f"flatten[{seed}]")
+
+
+CLEANUP_CASES = [(1, 0.02, 5), (2, 0.008, 3), (3, 0.05, 40)]
+
+
+def observe_cleanup(kind, seed, face_dist, min_neighbors):
     rng = np.random.default_rng(seed)
     v, t = _mc_like_mesh(rng, 400, 0.0)
     v, t = oracle_py.flatten_vertices(v, t, 1e-4, kind="port")       # cleanupMesh runs on the welded mesh in the program (:707-712)
-    va, ta = oracle_py.cleanup_mesh(v, t, face_dist, min_neighbors, kind="reference")
-    vb, tb = oracle_py.cleanup_mesh(v, t, face_dist, min_neighbors, kind="port")
-    assert len(ta) == len(tb) < len(t)
-    assert np.array_equal(va.view(np.uint32), vb.view(np.uint32)) and np.array_equal(ta, tb)
+    cv, ct = oracle_py.cleanup_mesh(v, t, face_dist, min_neighbors, kind=kind)
+    assert len(ct) < len(t)
+    return mesh_digests(cv, ct)
+
+
+@pytest.mark.parametrize("seed,face_dist,min_neighbors", CLEANUP_CASES)
+def test_cleanup_mesh_matches_the_reference_text(seed, face_dist, min_neighbors):
+    assert observe_cleanup("port", seed, face_dist, min_neighbors) == golden(f"cleanup[{seed}]")
+
+
+def observe_all(kind):
+    """Every observation above, keyed as in tests/golden/ref_pins.json."""
+    out = {}
+    for c in ORGANISE_CASES:
+        out[f"organise[{c[0]}]"] = observe_organise(kind, *c)
+    for c in FLATTEN_CASES:
+        out[f"flatten[{c[0]}]"] = observe_flatten(kind, *c)
+    for c in CLEANUP_CASES:
+        out[f"cleanup[{c[0]}]"] = observe_cleanup(kind, *c)
+    return out

@@ -4,7 +4,6 @@
 through the reference and records SHA-256 digests of its node dump, query results, render and
 mesh, plus a few scalar facts.  tests/test_golden.py replays the cases through the restatement
 (CPU) and the CUDA engine (GPU) and requires identical digests."""
-import hashlib
 import json
 import os
 import sys
@@ -14,7 +13,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 from cpu_tsdf_b200 import synth  # noqa: E402
-from tests.common import CAM, frames, query_points, canon_soup  # noqa: E402
+from tests.common import CAM, frames, query_points, canon_soup, sha  # noqa: E402
 
 CASES = {
     "c1_256_single": dict(cfg=dict(xres=256, yres=256, zres=256, cx=CAM.cx, cy=CAM.cy), scene="S1", n=1, stride=1, color=False, noise=None),
@@ -36,13 +35,6 @@ LONG_CASES = {
     "L3_256_static120": dict(cfg=dict(xres=256, yres=256, zres=256, cx=CAM.cx, cy=CAM.cy), scene="S1", n=120, stride=0, color=True, noise=9,
                              checkpoints=(60, 120), render_frames=(0,), render_ds=2, mesh_wmin=(2.0,)),
 }
-
-
-def sha(*arrays):
-    h = hashlib.sha256()
-    for a in arrays:
-        h.update(np.ascontiguousarray(a).tobytes())
-    return h.hexdigest()
 
 
 def run_case(vol_factory, case):
