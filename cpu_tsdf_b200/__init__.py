@@ -77,6 +77,7 @@ EXPORTS = [
     "b200tsdf_get_stats", "b200tsdf_download_nodes", "b200tsdf_download_color_payload", "b200tsdf_frustum_cull",
     "b200tsdf_profile_begin", "b200tsdf_profile_end",
     "b200tsdf_mesh_flatten", "b200tsdf_mesh_cleanup", "b200tsdf_mesh_free", "b200tsdf_meshpost_last_error", "b200tsdf_debug_timing",
+    "b200tsdf_voxel_centers", "b200tsdf_occupied_voxel_indices", "b200tsdf_is_empty",
 ]
 
 _lib = None
@@ -128,6 +129,9 @@ def load_library() -> C.CDLL:
     lib.b200tsdf_voxel_center.argtypes = [vp, C.c_int64, C.c_int64, C.c_int64, vp]
     lib.b200tsdf_voxel_index.argtypes = [vp, C.c_float, C.c_float, C.c_float, vp, vp]
     lib.b200tsdf_get_stats.argtypes = [vp, C.POINTER(Stats)]
+    lib.b200tsdf_voxel_centers.argtypes = [vp, C.c_int, C.POINTER(vp), C.POINTER(C.c_size_t)]
+    lib.b200tsdf_occupied_voxel_indices.argtypes = [vp, C.POINTER(vp), C.POINTER(C.c_size_t)]
+    lib.b200tsdf_is_empty.argtypes = [vp, C.POINTER(C.c_int32)]
     lib.b200tsdf_download_nodes.argtypes = [vp, vp, vp, vp, vp, vp, vp]; lib.b200tsdf_download_nodes.restype = C.c_int64
     lib.b200tsdf_download_color_payload.argtypes = [vp, vp]; lib.b200tsdf_download_color_payload.restype = C.c_int64
     lib.b200tsdf_frustum_cull.argtypes = [vp, vp, vp, vp]
@@ -452,6 +456,30 @@ class TSDFVolumeOctree:
         o = np.empty(3, np.int32); ins = np.zeros(1, np.int32)
         self._check(self._lib.b200tsdf_voxel_index(self._h, x, y, z, _ptr(o), _ptr(ins)))
         return bool(ins[0]), o
+
+    def _leaves(self, fn, dtype, *args) -> np.ndarray:
+        p, n = C.c_void_p(), C.c_size_t()
+        self._check(fn(self._h, *args, C.byref(p), C.byref(n)))
+        out = np.empty((n.value, 3), dtype)
+        if n.value:
+            C.memmove(out.ctypes.data, p.value, out.nbytes)
+        return out
+
+    def getVoxelCenters(self, nlevels: int = 4) -> np.ndarray:
+        """cpp:576-588 — centres of Octree::getLeaves (leaves, nlevels) as [n, 3] float32, in the reference's depth-first
+        order (nlevels = 0: the root; negative: every leaf)."""
+        return self._leaves(self._lib.b200tsdf_voxel_centers, np.float32, int(nlevels))
+
+    def getOccupiedVoxelIndices(self) -> np.ndarray:
+        """cpp:590-609 — getVoxelIndex of the centre of every leaf with w > 0 and |d| < 1, as [n, 3] int32 in the reference's
+        order (the reference appends them to a vector: concatenate to do the same)."""
+        return self._leaves(self._lib.b200tsdf_occupied_voxel_indices, np.int32)
+
+    def isEmpty(self) -> bool:
+        """h:283-287 — True from reset() until the first integrateCloud; load() takes the file's flag."""
+        out = C.c_int32()
+        self._check(self._lib.b200tsdf_is_empty(self._h, C.byref(out)))
+        return bool(out.value)
 
     def getFrustumCulledVoxels(self, trans):
         """cpp:619-652 — returns the boolean mask over the 8^coarse cells."""

@@ -403,6 +403,109 @@ __global__ void k_mesh_roots (Params gp, McParams mc, unsigned long long* __rest
   }
 }
 
+// ---- Octree::getLeaves: count pass (EMIT = false) and key pass over the stored levels >= C --------------------
+// warp-level compaction: one atomic per warp, keys land in emission order (hash layout), sorted afterwards
+template <bool EMIT>
+__device__ __forceinline__ void leaf_emit_warp (bool emit, unsigned long long key, unsigned long long* total, unsigned long long* keys)
+{
+  const unsigned m = __ballot_sync (0xffffffffu, emit);
+  if (!m) return;
+  const int lane = threadIdx.x & 31;
+  unsigned long long base = 0;
+  if (lane == 0) base = atomicAdd (total, (unsigned long long) __popc (m));
+  base = __shfl_sync (0xffffffffu, base, 0);
+  if (EMIT && emit) keys[base + __popc (m & ((1u << lane) - 1u))] = key;
+}
+
+// one warp per allocated brick; occupied: getOccupiedVoxelIndices' filter on top of getLeaves (leaves, -1)
+template <bool EMIT>
+__global__ void k_leaf_bricks (Params gp, int nlevels, int occupied, const int* __restrict__ list, int nbricks,
+                               unsigned long long* __restrict__ total, unsigned long long* __restrict__ keys)
+{
+  B2_STAGE_PARAMS (gp)
+  int warp = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  int lane = threadIdx.x & 31;
+  if (warp >= nbricks) return;
+  int slot = list[warp];
+  uint64_t key = p.keys[slot];
+  int t = (int) (key >> 60) - 1;
+  int bx = (int) ((key >> 40) & 0xFFFFF), by = (int) ((key >> 20) & 0xFFFFF), bz = (int) (key & 0xFFFFF);
+  int R = tier_root_level (p, t);
+  if (!brick_root_is_split (p, t, bx, by, bz)) return;         // nothing below an unsplit root exists
+  const uint32_t* sw = p.split + (size_t) slot * BRICK_SPLIT_WORDS;
+  for (int base = 0; base < BRICK_NODES; base += 32)
+  {
+    int i = base + lane;
+    bool emit = false; unsigned long long k = 0;
+    if (i < BRICK_NODES)
+    {
+      int kk = i < 8 ? 1 : (i < 72 ? 2 : 3);
+      int j = i - node_offset (kk);
+      int level = R + kk;
+      if (level >= p.C)                                          // levels above C are split by Octree::init: never stored leaves
+      {
+        // level C exists everywhere, the first level of a brick wherever its root is split (checked above); below, the parent's bit
+        bool exists = true;
+        if (kk > 1 && level > p.C) { int pj = j >> 3; exists = (sw[split_word_base (kk - 1) + (pj >> 5)] >> (pj & 31)) & 1; }
+        bool split = level < p.L && ((sw[split_word_base (kk) + (j >> 5)] >> (j & 31)) & 1);
+        emit = exists && leaf_emitted (level, split, nlevels);
+        if (emit && occupied) { float2 dw = p.nodes[(size_t) slot * BRICK_NODES + i]; emit = leaf_occupied (dw.x, dw.y); }
+        if (EMIT && emit)
+        {
+          int lx = 0, ly = 0, lz = 0;
+          for (int q = kk - 1; q >= 0; --q) { int c = (j >> (3 * q)) & 7; lx = (lx << 1) | (c >> 2); ly = (ly << 1) | ((c >> 1) & 1); lz = (lz << 1) | (c & 1); }
+          k = leaf_key (p, level, (bx << kk) | lx, (by << kk) | ly, (bz << kk) | lz);
+        }
+      }
+    }
+    leaf_emit_warp<EMIT> (emit, k, total, keys);
+  }
+}
+
+// the root arrays when they hold the coarse cells (Rtop == C)
+template <bool EMIT>
+__global__ void k_leaf_roots (Params gp, int nlevels, int occupied, unsigned long long* __restrict__ total, unsigned long long* __restrict__ keys)
+{
+  B2_STAGE_PARAMS (gp)
+  const int n = 1 << p.Rtop;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  bool emit = false; unsigned long long k = 0;
+  if (i < n * n * n && p.Rtop == p.C)
+  {
+    int z = i % n, y = (i / n) % n, x = i / (n * n);
+    emit = leaf_emitted (p.C, (p.root_split[i >> 5] >> (i & 31)) & 1, nlevels);
+    if (emit && occupied) { float2 dw = p.root_dw[i]; emit = leaf_occupied (dw.x, dw.y); }
+    if (EMIT && emit) k = leaf_key (p, p.C, x, y, z);
+  }
+  leaf_emit_warp<EMIT> (emit, k, total, keys);
+}
+
+// getLeaves (leaves, nlevels) for 0 <= nlevels <= C returns every node at level nlevels (all of them exist and the ones above C
+// are split), already in key order: the key of the i-th is i's bits moved up to the finest level
+__global__ void k_leaf_level (int L, int level, size_t count, unsigned long long* __restrict__ keys)
+{
+  size_t i = (size_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < count) keys[i] = ((unsigned long long) i << (3 * (L - level) + LEAF_LEVEL_BITS)) | (unsigned long long) level;
+}
+
+// key -> OctreeNode::getCenter (the float split accumulation) or, for occupied voxels, getVoxelIndex of that centre
+__global__ void k_leaf_decode (Params gp, const unsigned long long* __restrict__ keys, size_t count, float* __restrict__ xyz, int* __restrict__ ijk)
+{
+  B2_STAGE_PARAMS (gp)
+  size_t i = (size_t) blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= count) return;
+  int level, x, y, z;
+  leaf_decode (p, keys[i], level, x, y, z);
+  const float cx = center1d (p, level, x), cy = center1d (p, level, y), cz = center1d (p, level, z);
+  if (ijk)
+  {
+    int a, b, c;
+    (void) voxel_index (p, cx, cy, cz, a, b, c);                // the reference pushes the index whatever the bool says
+    ijk[3 * i] = a; ijk[3 * i + 1] = b; ijk[3 * i + 2] = c;
+  }
+  else { xyz[3 * i] = cx; xyz[3 * i + 1] = cy; xyz[3 * i + 2] = cz; }
+}
+
 } // namespace
 
 // ---------------------------------------------------------------------------------------------
@@ -533,6 +636,7 @@ struct b200tsdf
   }
   std::string err;
   float* mesh_v = nullptr; unsigned char* mesh_c = nullptr;
+  float* leaf_xyz = nullptr; int32_t* leaf_ijk = nullptr;   // last getVoxelCenters / getOccupiedVoxelIndices result (host)
   // grow-only device scratch for the read-side calls (queries, render): no allocation per call
   unsigned char* d_scratch = nullptr; size_t scratch_cap = 0;
   int scratch (size_t bytes)
@@ -711,6 +815,7 @@ void b200tsdf_destroy (b200tsdf_t* h)
   if (h->copy_stream) cudaStreamDestroy (h->copy_stream);
   if (h->gather_stream) cudaStreamDestroy (h->gather_stream);
   std::free (h->mesh_v); std::free (h->mesh_c);
+  std::free (h->leaf_xyz); std::free (h->leaf_ijk);
   delete h;
 }
 
@@ -1490,6 +1595,128 @@ int b200tsdf_mesh (b200tsdf_t* h, float w_min, int color_mode, float** verts, ui
 }
 
 void b200tsdf_free (void* p) { (void) p; /* mesh buffers are owned by the handle */ }
+
+} // extern "C"
+
+// ---- getVoxelCenters / getOccupiedVoxelIndices (tsdf_volume_octree.cpp:576-609) ---------------------------------
+// Octree::getLeaves on the device: a count pass and a key pass over the stored levels (one warp per brick, one thread per
+// root-array node), a radix sort of the keys into the order of the reference's depth-first walk, a decode pass into
+// centres or voxel indices, one copy to the host.  The node payload never leaves HBM: 12 bytes per returned node cross PCIe.
+namespace {
+struct DevMem
+{
+  void* p = nullptr;
+  ~DevMem () { cudaFree (p); }
+  template <typename T> T* as () const { return static_cast<T*> (p); }
+};
+
+// *out: host buffer of 3 values per node (float centres, or int32 indices when occupied), malloc'ed; *n: node count
+int leaves_on_device (b200tsdf* h, int nlevels, bool occupied, void** out, size_t* n)
+{
+  const char* what = occupied ? "getOccupiedVoxelIndices" : "getVoxelCenters";
+  if (!h->has_volume) return h->fail (B200TSDF_ESTATE, std::string (what) + " before reset()");
+  if (h->p.shard_count > 1)
+    return h->fail (B200TSDF_EINVAL, std::string (what) + " on a shard: the coarse cells it does not own are unsplit leaves here; "
+                    "gather the shards into one volume first (b200tsdf_gather_volume or b200tsdf_import_shard)");
+  cudaSetDevice (h->device);
+  if (int rc = pending_device_err (h)) return rc;
+  const Params& p = h->p;
+  cudaStream_t s = h->stream;
+  const int key_bits = 3 * p.L + LEAF_LEVEL_BITS;
+  size_t count = 0;
+  DevMem keys, sorted;
+  if (!occupied && nlevels >= 0 && nlevels <= p.C)
+  {
+    if (3 * nlevels >= 31) return h->fail (B200TSDF_ENOMEM, std::string (what) + ": more than 2^31 nodes requested");
+    count = (size_t) 1 << (3 * nlevels);
+    CK (cudaMalloc (&sorted.p, count * sizeof (unsigned long long)));
+    k_leaf_level<<<(unsigned) ((count + 255) / 256), 256, 0, s>>> (p.L, nlevels, count, sorted.as<unsigned long long> ());
+  }
+  else
+  {
+    if (occupied) nlevels = -1;                              // octree_->getLeaves (leaves): no level limit
+    DevMem list;
+    int* d_n = h->d_count + 40;
+    unsigned long long* d_total = h->d_stats + ST_SCRATCH;
+    CK (cudaMalloc (&list.p, h->pool * sizeof (int)));
+    CK (cudaMemsetAsync (d_n, 0, sizeof (int), s));
+    CK (cudaMemsetAsync (d_total, 0, sizeof (unsigned long long), s));
+    k_list_bricks<<<(unsigned) ((h->pool + 255) / 256), 256, 0, s>>> (p, list.as<int> (), d_n);
+    int nb = 0;
+    CK (cudaMemcpyAsync (&nb, d_n, sizeof (int), cudaMemcpyDeviceToHost, s));
+    CK (cudaStreamSynchronize (s));
+    const unsigned brick_blocks = (unsigned) (((size_t) nb * 32 + 127) / 128), root_blocks = (unsigned) ((h->root_n + 127) / 128);
+    if (nb) k_leaf_bricks<false><<<brick_blocks, 128, 0, s>>> (p, nlevels, occupied, list.as<int> (), nb, d_total, nullptr);
+    k_leaf_roots<false><<<root_blocks, 128, 0, s>>> (p, nlevels, occupied, d_total, nullptr);
+    unsigned long long total = 0;
+    CK (cudaMemcpyAsync (&total, d_total, sizeof (total), cudaMemcpyDeviceToHost, s));
+    CK (cudaStreamSynchronize (s));
+    if (total >= ((unsigned long long) 1 << 31)) return h->fail (B200TSDF_ENOMEM, std::string (what) + ": more than 2^31 nodes");
+    count = (size_t) total;
+    if (count)
+    {
+      CK (cudaMalloc (&keys.p, count * sizeof (unsigned long long)));
+      CK (cudaMalloc (&sorted.p, count * sizeof (unsigned long long)));
+      CK (cudaMemsetAsync (d_total, 0, sizeof (unsigned long long), s));
+      if (nb) k_leaf_bricks<true><<<brick_blocks, 128, 0, s>>> (p, nlevels, occupied, list.as<int> (), nb, d_total, keys.as<unsigned long long> ());
+      k_leaf_roots<true><<<root_blocks, 128, 0, s>>> (p, nlevels, occupied, d_total, keys.as<unsigned long long> ());
+      CK (cudaGetLastError ());
+      if (int e = b2_sort_keys (s, count, key_bits, keys.as<unsigned long long> (), sorted.as<unsigned long long> ()))
+        return h->fail (B200TSDF_ECUDA, std::string (what) + ": key sort failed: " + cudaGetErrorString ((cudaError_t) e));
+    }
+  }
+  CK (cudaGetLastError ());
+  *out = nullptr; *n = count;
+  if (!count) return check_device_err (h);
+  DevMem vals;
+  CK (cudaMalloc (&vals.p, count * 12));
+  k_leaf_decode<<<(unsigned) ((count + 255) / 256), 256, 0, s>>> (p, sorted.as<unsigned long long> (), count,
+                                                                  occupied ? nullptr : vals.as<float> (), occupied ? vals.as<int> () : nullptr);
+  CK (cudaGetLastError ());
+  void* host = std::malloc (count * 12);
+  if (!host) return h->fail (B200TSDF_ENOMEM, std::string (what) + ": host allocation failed");
+  cudaError_t e = cudaMemcpyAsync (host, vals.p, count * 12, cudaMemcpyDeviceToHost, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize (s);
+  if (e != cudaSuccess) { std::free (host); return h->fail (B200TSDF_ECUDA, std::string (what) + ": " + cudaGetErrorString (e)); }
+  h->d2h_bytes += (long long) (count * 12);
+  *out = host;
+  return check_device_err (h);
+}
+} // namespace
+
+extern "C" {
+
+int b200tsdf_voxel_centers (b200tsdf_t* h, int nlevels, float** xyz, size_t* n)
+{
+  if (!h || !xyz || !n) return B200TSDF_EINVAL;
+  void* out = nullptr; size_t cnt = 0;
+  int rc = leaves_on_device (h, nlevels, false, &out, &cnt);
+  if (rc) { std::free (out); return rc; }
+  std::free (h->leaf_xyz);
+  h->leaf_xyz = static_cast<float*> (out);
+  *xyz = h->leaf_xyz; *n = cnt;
+  return B200TSDF_OK;
+}
+
+int b200tsdf_occupied_voxel_indices (b200tsdf_t* h, int32_t** ijk, size_t* n)
+{
+  if (!h || !ijk || !n) return B200TSDF_EINVAL;
+  void* out = nullptr; size_t cnt = 0;
+  int rc = leaves_on_device (h, -1, true, &out, &cnt);
+  if (rc) { std::free (out); return rc; }
+  std::free (h->leaf_ijk);
+  h->leaf_ijk = static_cast<int32_t*> (out);
+  *ijk = h->leaf_ijk; *n = cnt;
+  return B200TSDF_OK;
+}
+
+int b200tsdf_is_empty (const b200tsdf_t* h, int32_t* out)
+{
+  if (!h || !out) return B200TSDF_EINVAL;
+  if (!h->has_volume) return B200TSDF_ESTATE;
+  *out = h->is_empty ? 1 : 0;
+  return B200TSDF_OK;
+}
 
 int b200tsdf_voxel_center (const b200tsdf_t* h, int64_t x, int64_t y, int64_t z, float* o)
 {

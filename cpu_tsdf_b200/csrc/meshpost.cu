@@ -373,3 +373,17 @@ int b2_sort_triangles (cudaStream_t s, size_t ntri, int key_bits, unsigned long 
   cudaFree (keys2); cudaFree (idx); cudaFree (idx2); cudaFree (tmp);
   return (int) e;
 }
+
+int b2_sort_keys (cudaStream_t s, size_t n, int key_bits, const unsigned long long* d_keys, unsigned long long* d_keys_out)
+{
+  if (!n) return 0;
+  if (n >= ((size_t) 1 << 31)) return (int) cudaErrorInvalidValue;
+  void* tmp = nullptr;
+  size_t bytes = 0;
+  cudaError_t e = cub::DeviceRadixSort::SortKeys (nullptr, bytes, d_keys, d_keys_out, (int) n, 0, key_bits, s);
+  if (e == cudaSuccess) e = cudaMalloc (&tmp, bytes);
+  if (e == cudaSuccess) e = cub::DeviceRadixSort::SortKeys (tmp, bytes, d_keys, d_keys_out, (int) n, 0, key_bits, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize (s);
+  cudaFree (tmp);
+  return (int) e;
+}

@@ -1176,6 +1176,36 @@ B2_HD unsigned long long mc_order_key (const Params& p, const NodePos& n)
   return k;
 }
 
+// ---- Octree::getLeaves (octree.cpp:99-109, 608-617) -----------------------------------------------
+// The nodes getLeaves returns never contain one another, so the order of its depth-first walk is the order of
+// mc_order_key.  The level sits in the low LEAF_LEVEL_BITS bits so that a key alone gives the node back (levels 0..19
+// need 5 bits): 3L + 5 significant bits.
+constexpr int LEAF_LEVEL_BITS = 5;
+B2_HD unsigned long long leaf_key (const Params& p, int level, int x, int y, int z)
+{
+  NodePos n; n.level = level; n.x = x; n.y = y; n.z = z;
+  return (mc_order_key (p, n) << LEAF_LEVEL_BITS) | (unsigned long long) level;
+}
+B2_HD void leaf_decode (const Params& p, unsigned long long key, int& level, int& x, int& y, int& z)
+{
+  level = (int) (key & ((1u << LEAF_LEVEL_BITS) - 1));
+  const unsigned long long m = key >> LEAF_LEVEL_BITS;
+  unsigned X = 0, Y = 0, Z = 0;
+  for (int l = 0; l < p.L; ++l)
+  {
+    X |= (unsigned) ((m >> (3 * l + 2)) & 1u) << l; Y |= (unsigned) ((m >> (3 * l + 1)) & 1u) << l; Z |= (unsigned) ((m >> (3 * l)) & 1u) << l;
+  }
+  x = (int) (X >> (p.L - level)); y = (int) (Y >> (p.L - level)); z = (int) (Z >> (p.L - level));
+}
+// Whether the walk of getLeaves (leaves, nlevels) returns an existing node at level >= 1: a child is pushed when it has no
+// children or when the level budget (nlevels - level) has reached 0; a negative budget never does.
+B2_HD bool leaf_emitted (int level, bool split, int nlevels)
+{
+  return nlevels < 0 ? !split : (level <= nlevels && (!split || level == nlevels));
+}
+// getOccupiedVoxelIndices (tsdf_volume_octree.cpp:598-601): w > 0 && fabs (d) < 1, fabs being the double one
+B2_HD bool leaf_occupied (float d, float w) { return w > 0 && fabs ((double) d) < 1; }
+
 // getGridValue (cpp:91-106)
 B2_HD float mc_grid_value (const Params& p, const McParams& mc, int x, int y, int z)
 {

@@ -225,6 +225,21 @@ int  b200tsdf_gather_volume (b200tsdf_t* h, b200tsdf_t* full, int root);
 int  b200tsdf_voxel_center (const b200tsdf_t* h, int64_t x, int64_t y, int64_t z, float* out3);
 int  b200tsdf_voxel_index (const b200tsdf_t* h, float x, float y, float z, int32_t* out3, int32_t* inside);
 
+/* ---- leaf enumeration: Octree::getLeaves (octree.cpp:99-109, 608-617) on the device ----------------------------
+ * Results come in the order of the reference's depth-first walk and are owned by the handle until the next call of the
+ * same entry point or b200tsdf_destroy.  Before the first reset () all three return B200TSDF_ESTATE.  On a handle created
+ * with shard_count > 1 the two enumerations return B200TSDF_EINVAL: the coarse cells it does not own are unsplit leaves
+ * there, so gather the shards into one volume first (b200tsdf_gather_volume / b200tsdf_import_shard). */
+/* TSDFVolumeOctree::getVoxelCenters (nlevels) (cpp:576-588): the centres of getLeaves (leaves, nlevels), 3 floats each.
+ * nlevels = 0 gives the root, a negative nlevels every leaf. */
+int  b200tsdf_voxel_centers (b200tsdf_t* h, int nlevels, float** xyz, size_t* n);
+/* TSDFVolumeOctree::getOccupiedVoxelIndices (cpp:590-609): getVoxelIndex of the centre of every leaf with w > 0 and
+ * |d| < 1, 3 int32 each.  The reference appends to the caller's vector; so does the C++ shim. */
+int  b200tsdf_occupied_voxel_indices (b200tsdf_t* h, int32_t** ijk, size_t* n);
+/* TSDFVolumeOctree::isEmpty (h:283-287): *out = 1 after reset () until the first integrateCloud, and whatever a loaded
+ * .vol says (cpp:239, 264) */
+int  b200tsdf_is_empty (const b200tsdf_t* h, int32_t* out);
+
 /* ---- introspection (tests, bench accounting) ------------------------------------------- */
 typedef struct b200tsdf_stats
 {

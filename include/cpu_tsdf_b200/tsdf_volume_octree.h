@@ -45,6 +45,7 @@ template <typename PointT> struct PointCloud
   bool is_dense = true;
   std::vector<PointT> points;
   typedef std::shared_ptr<PointCloud<PointT>> Ptr;
+  typedef std::shared_ptr<const PointCloud<PointT>> ConstPtr;
   const PointT& operator() (std::size_t column, std::size_t row) const { return points[row * width + column]; }
   std::size_t size () const { return points.size (); }
 };
@@ -54,6 +55,13 @@ struct Affine3d
   static Affine3d Identity () { return Affine3d (); }
   const double* data () const { return m; }
 };
+// Eigen::Vector3i as getOccupiedVoxelIndices uses it: idx (0), idx (1), idx (2)
+struct Vector3i
+{
+  int v[3] = { 0, 0, 0 };
+  int& operator() (int i) { return v[i]; }
+  int operator() (int i) const { return v[i]; }
+};
 struct TriangleSoup { std::vector<float> xyz; std::vector<std::uint8_t> rgb; std::vector<std::int32_t> polygons; };
 struct PointXYZRGBNormal { float x, y, z, pad = 1.f; float normal_x, normal_y, normal_z, npad = 0.f; std::uint8_t b = 0, g = 0, r = 0, a = 255; float curvature = 0.f, cpad[2] = { 0.f, 0.f }; };
 #else
@@ -62,6 +70,7 @@ using pcl::PointCloud;
 using pcl::PointNormal;
 using pcl::PointXYZ;
 typedef Eigen::Affine3d Affine3d;
+typedef Eigen::Vector3i Vector3i;
 #endif
 
 namespace detail
@@ -245,6 +254,36 @@ public:
   { float o[3] = { 0, 0, 0 }; b200tsdf_voxel_center (h_, (std::int64_t) x, (std::int64_t) y, (std::int64_t) z, o); PointXYZ p; p.x = o[0]; p.y = o[1]; p.z = o[2]; return p; }
   bool getVoxelIndex (float x, float y, float z, int& x_i, int& y_i, int& z_i) const               // cpp:562-574
   { std::int32_t o[3] = { 0, 0, 0 }, in = 0; b200tsdf_voxel_index (h_, x, y, z, o, &in); x_i = o[0]; y_i = o[1]; z_i = o[2]; return in != 0; }
+
+  // cpp:576-588: the centres of Octree::getLeaves (leaves, nlevels) in the reference's order, as a cloud of width n and
+  // height 1 (nlevels = 0: the root; negative: every leaf).  Empty when the call fails (status () tells why).
+  typename PointCloud<PointXYZ>::ConstPtr getVoxelCenters (int nlevels = 4) const
+  {
+    typename PointCloud<PointXYZ>::Ptr cloud (new PointCloud<PointXYZ>);
+    float* xyz = nullptr; std::size_t n = 0;
+    status_ = h_ ? b200tsdf_voxel_centers (h_, nlevels, &xyz, &n) : B200TSDF_ENODEVICE;
+    if (status_ != 0) n = 0;
+    cloud->points.resize (n);
+    cloud->width = static_cast<std::uint32_t> (n); cloud->height = 1;
+    for (std::size_t i = 0; i < n; ++i) { PointXYZ& p = cloud->points[i]; p.x = xyz[3 * i]; p.y = xyz[3 * i + 1]; p.z = xyz[3 * i + 2]; }
+    return cloud;
+  }
+  // cpp:590-609: appends getVoxelIndex of the centre of every leaf with w > 0 and |d| < 1, as the reference does
+  void getOccupiedVoxelIndices (std::vector<Vector3i>& indices) const
+  {
+    std::int32_t* ijk = nullptr; std::size_t n = 0;
+    status_ = h_ ? b200tsdf_occupied_voxel_indices (h_, &ijk, &n) : B200TSDF_ENODEVICE;
+    if (status_ != 0) return;
+    indices.reserve (indices.size () + n);
+    for (std::size_t i = 0; i < n; ++i) { Vector3i idx; idx (0) = ijk[3 * i]; idx (1) = ijk[3 * i + 1]; idx (2) = ijk[3 * i + 2]; indices.push_back (idx); }
+  }
+  // h:283-287: true from reset () until the first integrateCloud; load () takes the file's flag
+  bool isEmpty () const
+  {
+    std::int32_t e = 1;
+    if (h_) b200tsdf_is_empty (h_, &e);
+    return e != 0;
+  }
 
   // TSDFInterface::instantiateFromFile (src/lib/tsdf_interface.cpp:44-51): "for now everything is an octree"
   static Ptr instantiateFromFile (const std::string& filename, int device = 0, int pool_log2 = 0)
